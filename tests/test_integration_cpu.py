@@ -4,13 +4,17 @@
   ape/layers/multi_scale_deform_attn.py:415-423): with it in place the reference module file defines the real
   MultiScaleDeformableAttention class and finds `torch.ops.ape.ms_deform_attn_forward`.
 * every `_target_` override INTEGRATION.md tells a user to pass names a node of the reference's own LazyConfig tree
-  (configs/…/ape_deta_vitl_eva02_clip_vlf_lsj1024_cp_16x4_1080k.py and the files it builds on), parsed with `ast` (detectron2
-  is not installed here), and the engine class behind it accepts every keyword the config passes to the reference class.
+  (configs/…/ape_deta_vitl_eva02_clip_vlf_lsj1024_cp_16x4_1080k.py and the files it builds on), and the engine class behind
+  it accepts every keyword the config passes to the reference class.
 * `Instances.to_detectron2()` maps the fields onto detectron2's types.
-* entity gates and thing-class slicing of the instance branch (deformable_detr_segm_vl.py:575-593)."""
-import ast
+* entity gates and thing-class slicing of the instance branch (deformable_detr_segm_vl.py:575-593).
+
+What the reference imports and calls, and its config tree (parsed with `ast`: detectron2 is not installed), are recorded in
+tests/golden/reference_integration.json by tests/golden/gen_reference_golden.py."""
+import importlib
 import importlib.util
 import inspect
+import json
 import os
 import re
 import sys
@@ -19,9 +23,14 @@ import types
 import pytest
 import torch
 
+from conftest import GOLDEN
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
-needs_ref = pytest.mark.skipif(not os.path.isdir(REF), reason="the reference checkout only exists in the build container")
+
+
+def _reference():
+    with open(os.path.join(GOLDEN, "reference_integration.json")) as f:
+        return json.load(f)
 
 
 def _load(path, name):
@@ -31,20 +40,21 @@ def _load(path, name):
     return mod
 
 
-@needs_ref
 def test_shipped_C_shim_satisfies_the_reference_import_contract(built):
-    saved = {k: sys.modules.get(k) for k in ("ape", "ape._C", "ape.layers", "ape.layers.multi_scale_deform_attn")}
+    ref = _reference()
+    assert ref["msda_module_imports_from_ape"] == ["_C"]  # the module's only import from the package: its `try` guard
+    assert "ms_deform_attn_forward" in ref["msda_module_ops"]
+    saved = {k: sys.modules.get(k) for k in ("ape", "ape._C")}
     try:
         pkg = types.ModuleType("ape")
-        pkg.__path__ = [os.path.join(REF, "ape")]
+        pkg.__path__ = [os.path.join(ROOT, "integration", "ape")]
         sys.modules["ape"] = pkg
-        shim = _load(os.path.join(ROOT, "integration", "ape", "_C.py"), "ape._C")
-        sys.modules["ape._C"] = shim
-        pkg._C = shim
-        ref = _load(os.path.join(REF, "ape", "layers", "multi_scale_deform_attn.py"), "ape.layers.multi_scale_deform_attn")
-        assert inspect.isclass(ref.MultiScaleDeformableAttention) and issubclass(ref.MultiScaleDeformableAttention, torch.nn.Module)
-        m = ref.MultiScaleDeformableAttention(embed_dim=64, num_heads=4, num_levels=2, num_points=4)  # dummy class would raise ImportError
-        assert hasattr(m, "sampling_offsets")
+        sys.modules.pop("ape._C", None)
+        ns = {}
+        exec("from ape import _C", ns)  # the statement the reference's module runs; ImportError would select its dummy class
+        assert ns["_C"].__file__ == os.path.join(ROOT, "integration", "ape", "_C.py")
+        for op in ref["msda_module_ops"]:
+            assert hasattr(torch.ops.ape, op), f"the reference calls torch.ops.ape.{op}, which the shim does not register"
         schema = str(torch.ops.ape.ms_deform_attn_forward.default._schema)
         assert "Tensor value, Tensor spatial_shapes, Tensor level_start_index, Tensor sampling_loc, Tensor attn_weight, int im2col_step" in schema
         with pytest.raises(RuntimeError, match="Not implemented on the CPU"):  # ms_deform_attn.h:39
@@ -59,75 +69,9 @@ def test_shipped_C_shim_satisfies_the_reference_import_contract(built):
                 sys.modules[k] = v
 
 
-# ---- LazyConfig tree from the config sources -----------------------------------------------------------------------
-LEAF = "<value>"
-
-
-def _lazy_tree(node, env):
-    """`L(Target)(kw=...)` -> {"_target_": "Target", kw: subtree | LEAF}; a bare name bound to a tree -> that tree."""
-    if isinstance(node, ast.Call) and isinstance(node.func, ast.Call) and getattr(node.func.func, "id", "") == "L":
-        tgt = node.func.args[0]
-        name = tgt.id if isinstance(tgt, ast.Name) else ast.unparse(tgt)
-        return {"_target_": name, **{kw.arg: _lazy_tree(kw.value, env) for kw in node.keywords if kw.arg}}
-    if isinstance(node, ast.Name) and isinstance(env.get(node.id), dict):
-        return env[node.id]
-    return LEAF
-
-
-def _attr_path(t):
-    path = []
-    while isinstance(t, ast.Attribute):
-        path.append(t.attr)
-        t = t.value
-    return (t.id if isinstance(t, ast.Name) else None), path[::-1]
-
-
-def _run_config(src, env):
-    """The three statement forms the configs use to build the model tree: `name = L(..)(..)`,
-    `name.a.b = <L-call | value>` and `name.a.b.update(_target_=X, ...)`."""
-    for stmt in ast.parse(src).body:
-        if isinstance(stmt, ast.Assign) and len(stmt.targets) == 1:
-            tgt = stmt.targets[0]
-            if isinstance(tgt, ast.Name):
-                tree = _lazy_tree(stmt.value, env)
-                if isinstance(tree, dict):
-                    env[tgt.id] = tree
-                continue
-            root, path = _attr_path(tgt)
-            node = env.get(root)
-            for k in path[:-1]:
-                node = node.get(k) if isinstance(node, dict) else None
-            if isinstance(node, dict) and path:
-                node[path[-1]] = _lazy_tree(stmt.value, env)
-        elif isinstance(stmt, ast.Expr) and isinstance(stmt.value, ast.Call) and isinstance(stmt.value.func, ast.Attribute) \
-                and stmt.value.func.attr == "update":
-            root, path = _attr_path(stmt.value.func.value)
-            node = env.get(root)
-            for k in path:
-                node = node.get(k) if isinstance(node, dict) else None
-            if isinstance(node, dict):
-                for kw in stmt.value.keywords:
-                    if kw.arg == "_target_":
-                        node["_target_"] = kw.value.id if isinstance(kw.value, ast.Name) else ast.unparse(kw.value)
-                    elif kw.arg:
-                        node[kw.arg] = _lazy_tree(kw.value, env)
-
-
-def _reference_model_tree():
-    env = {}
-    for rel in ("configs/common/backbone/vitl_eva02_clip.py",
-                "configs/COCO_InstanceSegmentation/ape_deta/models/ape_deta_r50.py",
-                "configs/LVISCOCOCOCOSTUFF_O365_OID_VGR_SA1B_REFCOCO_GQA_PhraseCut_Flickr30k/ape_deta/"
-                "ape_deta_vitl_eva02_clip_vlf_lsj1024_cp_16x4_1080k.py"):
-        _run_config(open(os.path.join(REF, rel)).read(), env)
-    tree = env["model"]
-    assert tree["_target_"] == "SomeThing" and tree["model_vision"]["_target_"] == "DeformableDETRSegmVL"
-    return tree
-
-
-@needs_ref
 def test_integration_target_overrides_name_real_config_nodes(built):
-    tree = _reference_model_tree()
+    tree = _reference()["model_tree"]
+    assert tree["_target_"] == "SomeThing" and tree["model_vision"]["_target_"] == "DeformableDETRSegmVL"
     text = open(os.path.join(ROOT, "INTEGRATION.md")).read()
     overrides = re.findall(r"(model(?:\.\w+)+)\._target_=(ape_b200(?:\.\w+)+)", text)
     assert len(overrides) >= 9

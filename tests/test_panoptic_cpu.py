@@ -1,22 +1,23 @@
 """CPU: the vectorised panoptic merging (ape_b200/modeling/postprocess.py) against the reference's own
-`DeformableDETRSegmVL._postprocess_panoptic` (deformable_detr_segm_vl.py:919-998) executed unmodified under the import
-shims — identical segment maps and segments_info on random predictions (build container only)."""
+`DeformableDETRSegmVL._postprocess_panoptic` (deformable_detr_segm_vl.py:919-998) — identical segment maps and segments_info
+on random predictions.  The reference's results were recorded by tests/golden/gen_reference_golden.py, which executes that
+function unmodified under the import shims."""
+import json
+import os
 import types
 
+import numpy as np
 import pytest
 import torch
 
 from ape_b200.modeling.postprocess import postprocess_panoptic
+from conftest import GOLDEN
+
+CASES = [(0, 12, 9, False), (1, 40, 7, True), (2, 3, 5, False), (3, 25, 12, True)]
 
 
-@pytest.mark.parametrize("seed,K,n_cls,stuff_first", [(0, 12, 9, False), (1, 40, 7, True), (2, 3, 5, False), (3, 25, 12, True)])
-def test_equals_reference_function(seed, K, n_cls, stuff_first):
-    from oracle import refshim
-
-    if not refshim.available():
-        pytest.skip("reference sources not present (GPU box)")
-    refshim.install()
-    segm = refshim.load("ape.modeling.ape_deta.deformable_detr_segm_vl")
+def panoptic_case(seed, K, n_cls, stuff_first):
+    """Seeded predictions and the metadata / config the reference function takes."""
     g = torch.Generator().manual_seed(seed)
     H = W = 48
     image_size, out_hw = (40, 44), (80, 88)
@@ -35,9 +36,16 @@ def test_equals_reference_function(seed, K, n_cls, stuff_first):
     meta.get = lambda key, default=None: getattr(meta, key, default)
     cfg = dict(prob=0.5, pano_temp=0.06, transform_eval=True, object_mask_threshold=0.3, overlap_threshold=0.6)
     images = types.SimpleNamespace(image_sizes=[image_size])
-    want = segm.DeformableDETRSegmVL._postprocess_panoptic([mask_cls], [mask_pred], [{"height": out_hw[0], "width": out_hw[1]}],
-                                                          images, meta, cfg)[0]["panoptic_seg"]
+    return mask_cls, mask_pred, image_size, out_hw, meta, cfg, images
+
+
+@pytest.mark.parametrize("seed,K,n_cls,stuff_first", CASES)
+def test_equals_reference_function(seed, K, n_cls, stuff_first):
+    mask_cls, mask_pred, image_size, out_hw, _, cfg, _ = panoptic_case(seed, K, n_cls, stuff_first)
+    gold = np.load(os.path.join(GOLDEN, "panoptic_reference.npz"))
+    want_seg, want_info = torch.from_numpy(gold[f"seg{seed}"]), json.loads(str(gold[f"info{seed}"]))
+    n_thing = n_cls // 2
     seg, info = postprocess_panoptic(mask_cls, mask_pred, image_size, out_hw[0], out_hw[1], range(n_thing), n_thing, stuff_first, cfg)
-    assert torch.equal(seg, want[0])
-    assert info == want[1]
+    assert torch.equal(seg, want_seg)
+    assert info == want_info
     assert len(info) > 0 or K < 4
